@@ -9,6 +9,8 @@ Contract (see the task statement): `python bench.py --gpus N --steps K --warmup 
   vq           : the second headline metric (VQ argmin GB/s, algorithmic bytes) measured live
   cpu_baseline : the CPU oracle (a restatement of the reference; kind "port") timed on this box's host cores
 `--impl reference` times that same CPU implementation alone and prints the line with "impl": "reference".
+`--dump-outputs DIR` writes what the last timed step computed (dump_outputs) so that two builds can be compared output for
+output: model, weights and batch come from fixed seeds, so the same arguments give the same inputs on every run.
 Workload = BASELINE.json configs[1]; synthetic data (torch.rand images, seeded default-init weights, N(0,1) codebook,
 q_counter past the re-init window so the real VQ branch runs — SURVEY.md 8d). Proxy loss: L1 + codebook term.
 """
@@ -113,10 +115,11 @@ def cpu_threads():
     return n
 
 
-def cpu_reference_steps(steps, warmup, batch=2):
-    """The reference's own CPU implementation of the path, all host threads, on a bounded sample of the workload (`batch`
-    images per step instead of 32). kind "reference": the UNMODIFIED reference modules staged under oracle/_ref
-    (oracle/vendor_ref.py; BASELINE.md section 3); kind "port": the oracle restatement, when oracle/_ref is absent."""
+def cpu_reference_steps(steps, warmup, batch=2, budget=None):
+    """The reference's own CPU implementation of the path, all host threads, on a sample of the workload (`batch` images
+    per step instead of 32); with `budget` (seconds) the timed steps stop once they exceed it. kind "reference": the
+    UNMODIFIED reference modules staged under oracle/_ref (oracle/vendor_ref.py; BASELINE.md section 3); kind "port": the
+    oracle restatement, when oracle/_ref is absent."""
     from oracle import vendor_ref
     cores = cpu_threads()
     x = torch.rand(batch, 3, RES, RES, generator=torch.Generator().manual_seed(1234))
@@ -148,16 +151,13 @@ def cpu_reference_steps(steps, warmup, batch=2):
             dec, diff, _ = O.vqbase_forward(sd, IMG_CFG, x)
             O.proxy_loss(x, dec, diff).backward()
     times = []
-    budget = float(os.environ.get("MAS_CPU_ARM_SECONDS", "60"))   # bounded sample: stop once the timed steps exceed this
-    warmup = min(warmup, 1)
-    steps = min(steps, 5)
     for i in range(warmup + steps):
         t0 = time.perf_counter()
         one()
         dt = time.perf_counter() - t0
         if i >= warmup:
             times.append(dt)
-            if sum(times) > budget:
+            if budget is not None and sum(times) > budget:
                 break
     return dict(value=batch * len(times) / sum(times), sec=sum(times) / len(times), done=len(times), kind=kind, cores=cores,
                 batch=batch)
@@ -169,7 +169,7 @@ def run_reference(args, rank):
     r = cpu_reference_steps(args.steps, args.warmup, batch=2)
     v = r["value"]
     line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "images/s", "n_gpus": args.gpus, "steps": r["done"],
-            "warmup": min(args.warmup, 1), "ms_per_step": r["sec"] * 1e3, "higher_is_better": True, "scaling": "weak",
+            "warmup": args.warmup, "ms_per_step": r["sec"] * 1e3, "higher_is_better": True, "scaling": "weak",
             "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": {"workload": "VQ-IMG 256x256 codebook=8192 dim=256 (BASELINE configs[1])",
                        "sample": "%d images per step (the batch-32 workload sampled at batch %d)" % (r["batch"], r["batch"])},
@@ -408,6 +408,44 @@ def transformer_metric(dev, pk, batch=8, steps=3, warmup=2):
             "kernel_rooflines": roofs}
 
 
+DUMP_MAX_ELEMS = 8 << 20       # per output array: a larger one is written as a fixed, seeded sample of this many elements
+GRAD_SAMPLE = 4096             # elements sampled from each parameter gradient larger than this
+
+
+def _seeded_sample(t, k, seed):
+    """`k` elements of `t` (flattened) at indices drawn from a fixed seed, in ascending order; all of `t` if it is smaller."""
+    t = t.detach().reshape(-1)
+    if t.numel() <= k:
+        return t
+    idx = torch.randint(0, t.numel(), (k,), generator=torch.Generator().manual_seed(seed)).sort().values
+    return t[idx.to(t.device)]
+
+
+def dump_outputs(out_dir, model, last):
+    """Writes what the last timed step returned to its caller, as float32 / float64 .npy files under `out_dir`: the
+    reconstruction `dec` (whole, or `dec_sample` when larger than DUMP_MAX_ELEMS), the codebook term `diff`, the `loss`,
+    `grad_norms` (float64 L2 norm of every parameter gradient, model.named_parameters() order) and `grad_sample` (per
+    parameter in that order, up to GRAD_SAMPLE gradient elements at seeded indices, concatenated). On a B200, two runs of
+    one build give bit-identical dec / diff / loss; the weight gradients differ in the last bits (reduction order), so
+    compare them with a tolerance."""
+    import numpy as np
+    dec = last["dec"].detach()
+    dec_name, dec = ("dec", dec) if dec.numel() <= DUMP_MAX_ELEMS else ("dec_sample", _seeded_sample(dec, DUMP_MAX_ELEMS, 0))
+    arrays = {dec_name: dec.float(), "diff": last["diff"].detach().float(), "loss": last["loss"].detach().float()}
+    named = [(k, p.grad) for k, p in model.named_parameters()]
+    missing = [k for k, g in named if g is None]
+    assert not missing, "parameters without a gradient after the timed step: %s" % missing[:5]
+    arrays["grad_norms"] = torch.stack([g.detach().double().norm() for _, g in named])
+    arrays["grad_sample"] = torch.cat([_seeded_sample(g, GRAD_SAMPLE, i).float() for i, (_, g) in enumerate(named)])
+    arrays = {k: t.contiguous().cpu().numpy() for k, t in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= 64 << 20, "dumped outputs exceed 64 MB (%d bytes)" % total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return sorted(arrays)
+
+
 def _fmt():
     from mas_b200 import ops
     return "fp16 (3x3 convolutions) / tf32 (1x1)" if ops.get_operand_format() == "f16" else "tf32"
@@ -428,7 +466,11 @@ def main():
                     help="skip the per-kernel blocks (roofline / VQ sweep / AttnBlock / CPU baseline): launch-list captures under ncu")
     ap.add_argument("--graph", action="store_true",
                     help="single GPU: replay the step from one CUDA graph (mas_b200.graph.GraphedStep) instead of launching from Python")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's outputs and gradients as .npy files to DIR (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -457,6 +499,7 @@ def main():
     else:
         img_host = torch.rand(B, 3, RES, RES, generator=gen).pin_memory()
     img_dev = img_host.to(dev)
+    last = {}       # the outputs of the latest step, kept only for --dump-outputs
 
     def step(img):
         net.zero_grad(set_to_none=True)
@@ -467,6 +510,8 @@ def main():
         else:
             loss = (img - dec).abs().mean() + diff
         loss.backward()
+        if args.dump_outputs:
+            last.update(dec=dec, diff=diff, loss=loss)
         return loss
 
     def timed(fn, warmup, steps):
@@ -499,6 +544,8 @@ def main():
 
         def loss_fn(m, x):
             dec, diff = m(x)
+            if args.dump_outputs:     # during capture: these become the graph's static output buffers
+                last.update(dec=dec, diff=diff)
             if seg:
                 from mas_b200 import ops
                 return ops.BCELogitsFn.apply(dec, x, pos_w) + diff
@@ -517,6 +564,10 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     if gs is not None:
         launches = gs.launches_per_step * args.steps
+        last["loss"] = gs.loss
+    if args.dump_outputs and rank == 0:
+        print("outputs of the last timed step written to %s: %s" % (args.dump_outputs, ", ".join(dump_outputs(args.dump_outputs, model, last))),
+              file=sys.stderr)
 
     def e2e_step():
         if gs is not None:
@@ -582,7 +633,7 @@ def main():
         except Exception as e:  # noqa: BLE001
             line["transformer"] = {"error": str(e)[:200]}
     if not args.no_cpu_baseline and world == 1:   # reported baseline: rank 0 at N=1 only
-        r = cpu_reference_steps(3, 1, batch=2)
+        r = cpu_reference_steps(3, 1, batch=2, budget=float(os.environ.get("MAS_CPU_ARM_SECONDS", "60")))
         line["cpu_baseline"] = {"value": r["value"], "unit": "images/s", "cores": r["cores"], "kind": r["kind"],
                                 "sample": "%d timed fwd+bwd steps of %d images after 1 warm-up (%.1f s/step)" % (r["done"], r["batch"], r["sec"])}
     print(json.dumps(line), flush=True)

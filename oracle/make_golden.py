@@ -58,6 +58,8 @@ def main():
         tensor_path_block_fixtures(M)
     if only is None or "img256" in only:
         img256_fixture(ref_models)
+    if only is None or "codebook" in only:
+        codebook_schedule_fixture(M)
 
 
 def base_fixtures(ref_models, M, V, L, T):
@@ -308,6 +310,27 @@ def img256_fixture(ref_models):
                     grad_norms={k: float(p.grad.double().norm()) for k, p in named.items()}, grad_samples=grad_samples),
                os.path.join(OUT, "vqbase_img_256.pt"))
     print("img 256 done: loss", float(loss))
+
+
+def codebook_schedule_fixture(M):
+    """G9: the REAL reference's Codebook through its warm-up steps 1 .. q_init - 1 (init_steps 4: collects from step 5,
+    quantises from step 12): per step the output, loss, indices, counter and reservoir, under the same global seeds as
+    tests/test_host_logic_vq_cpu.py replays them (reservoir sampling draws two torch.randperm per step)."""
+    K, D, init_steps = 16, 8, 4
+    torch.manual_seed(3)
+    cb = M.Codebook(K, D, 0.25, init_steps, 60)
+    cb.train()
+    gz = torch.Generator().manual_seed(11)
+    zs = [torch.randn(3, D, 4, 4, generator=gz) for _ in range(16)]
+    steps = []
+    for step, z in enumerate(zs[:11], start=1):
+        torch.manual_seed(100 + step)
+        z_q, loss, idx = cb(z)
+        steps.append(dict(z_q=z_q.detach().clone(), loss=float(loss), idx=idx, q_counter=cb.q_counter,
+                          reservoir=None if cb.reservoir is None else cb.reservoir.clone()))
+    torch.save(dict(K=K, D=D, init_steps=init_steps, reservoir_size=60, weight=cb.embedding.weight.detach().clone(), steps=steps),
+               os.path.join(OUT, "codebook_schedule.pt"))
+    print("codebook schedule done")
 
 
 if __name__ == "__main__":

@@ -839,32 +839,28 @@ def test_codebook_schedule_host_logic_against_the_reference(vq_emu):
     same two torch.randperm draws per step), warm-up bypass - step by step IDENTICAL to the real reference's Codebook under the
     same seed up to the first re-initialisation; then our k-means replacement (the reference calls the absent
     fast_pytorch_kmeans there): triggered on the reference's schedule, lowers the quantisation error, and the following steps
-    quantise against the new centres."""
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), ".."))
-    from oracle import vendor_ref
-    if not vendor_ref.available():
-        pytest.skip("oracle/_ref not staged (needs /root/reference once)")
+    quantise against the new centres. The reference's per-step results are tests/golden/codebook_schedule.pt
+    (oracle/make_golden.py --only=codebook)."""
     from models import modules as M
-    R = vendor_ref.load_models().modules
+    g = torch.load(os.path.join(GOLDEN, "codebook_schedule.pt"), weights_only=False)
     K, D, init_steps = 16, 8, 4                                  # collect from step 5, quantise from step 12, re-init every 2 steps
+    assert (g["K"], g["D"], g["init_steps"], g["reservoir_size"]) == (K, D, init_steps, 60)
     torch.manual_seed(3)
-    ours, ref = M.Codebook(K, D, 0.25, init_steps, 60), R.Codebook(K, D, 0.25, init_steps, 60)
-    ref.load_state_dict(ours.state_dict())
-    ours.train(); ref.train()
+    ours = M.Codebook(K, D, 0.25, init_steps, 60)
+    assert torch.equal(ours.embedding.weight.detach(), g["weight"])    # same initial codes as the reference's under that seed
+    ours.train()
     gz = torch.Generator().manual_seed(11)
     zs = [torch.randn(3, D, 4, 4, generator=gz) for _ in range(16)]
     for step, z in enumerate(zs[:11], start=1):                  # steps 1 .. q_init - 1: both bypass, both collect from step 5 on
         torch.manual_seed(100 + step)
         a = ours(z)
-        torch.manual_seed(100 + step)
-        b = ref(z)
-        assert ours.q_counter == ref.q_counter == step
-        assert a[2] is None and b[2] is None and float(a[1]) == 0.0 and torch.equal(a[0], b[0])
+        b = g["steps"][step - 1]
+        assert ours.q_counter == b["q_counter"] == step
+        assert a[2] is None and b["idx"] is None and float(a[1]) == 0.0 == b["loss"] and torch.equal(a[0], b["z_q"])
         if step > init_steps:
-            assert torch.equal(ours.reservoir, ref.reservoir) and ours.reservoir.shape[0] == min(60, 30 * (step - init_steps))
+            assert torch.equal(ours.reservoir, b["reservoir"]) and ours.reservoir.shape[0] == min(60, 30 * (step - init_steps))
         else:
-            assert ours.reservoir is None and ref.reservoir is None
+            assert ours.reservoir is None and b["reservoir"] is None
     assert "mas_vq_forward" not in vq_emu.names
     # step q_init = 12: the first re-initialisation from the reservoir, then quantisation
     e0 = ours.embedding.weight.detach().clone()
